@@ -22,6 +22,10 @@ work is fixed as N grows.
           every key row, two heads, fp32 read-out; max relative Frobenius error over ranks (north_star bound 1e-3)
   reference_probe   whether the reference's own JAX implementation (jax + the un-vendored `ringattention` package)
           is importable on this box — if it ever is, the oracle is pinned against it on a small case right here
+
+--dump-outputs DIR writes what the last timed step returned to its caller (out, dq, dk, dv) as float32 .npy files, a
+fixed seeded sample of token rows (see dump_outputs), so that two builds can be compared output for output: the inputs
+depend only on the arguments.
 """
 import argparse
 import json
@@ -293,6 +297,24 @@ def bench_vqgan(dev, peaks, world, rank, with_cpu=True):
     return rec
 
 
+DUMP_ROWS = 512     # token rows sampled per output: 4 outputs x 512 rows x 32 heads x 128 x fp32 = 32 MB
+
+
+def dump_outputs(dirname, outputs, rank, world):
+    """Write the step's outputs ([1, S/N, H, D] each, 1 GiB apiece at 128K tokens on one GPU) as DIR/<name>.npy, float32,
+    shape [rows, H, D]: the same seeded sample of DUMP_ROWS token rows of the local shard (sorted, every head and channel)
+    in every run. With N ranks each writes DUMP_ROWS / N rows of its own shard as <name>_rank<r>.npy."""
+    import numpy as np
+    import torch
+    os.makedirs(dirname, exist_ok=True)
+    g = torch.Generator().manual_seed(0)
+    rows = torch.randperm(outputs[0].shape[1], generator=g)[:max(1, DUMP_ROWS // world)].sort().values
+    suffix = "" if world == 1 else "_rank%d" % rank
+    for name, t in zip(("out", "dq", "dk", "dv"), outputs):
+        a = t.detach()[0].index_select(0, rows.to(t.device)).float().cpu().numpy()
+        np.save(os.path.join(dirname, name + suffix + ".npy"), a)
+
+
 # ------------------------------------------------------------------------------------------------
 def main():
     ap = argparse.ArgumentParser()
@@ -310,7 +332,11 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-parity", action="store_true", help="(debug) skip the oracle check that precedes the timing")
     ap.add_argument("--no-vqgan", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write a fixed sample of the last timed step's out / dq / dk / dv to DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -401,12 +427,17 @@ def main():
     barrier()
     calls0 = _lib.launch_count()
     t0.record()
-    for _ in range(K):
-        step()
+    for i in range(K):
+        last = step()
+        if i + 1 < K:
+            last = None         # only the last step's results outlive their step
     t1.record()
     barrier()
     gpu_launches = _lib.launch_count() - calls0      # C-ABI compute calls of this rank in the timed region
     ms = t0.elapsed_time(t1) / K
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, last, rank, world)
+    last = None
     clocks = sampler.stop() if rank == 0 else None
     if world > 1:
         tm = torch.tensor([ms], device=dev)
@@ -526,7 +557,7 @@ def main():
         keep[0] = keep[1] = None
 
     e2e_step()
-    n_e2e = max(3, min(K, 6))
+    n_e2e = K
     if not args.e2e_serial:
         e2e_setup()
         e2e_pipelined(2)            # warm-up of the pipelined path (untimed)

@@ -3,14 +3,11 @@ prologue and the vision token framing. The oracles are checked against fixtures 
 own functions (tools/make_golden_next_rows_from_reference.py), and the numerical design of the CUDA kernel (angles
 rebuilt from 64 inverse frequencies, cos/sin rounded once from double) is checked against the reference's table."""
 import os
-import subprocess
-import sys
 
 import numpy as np
 import pytest
 
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 TAGS = ("t1e4", "t5e7")
 
 
@@ -90,21 +87,6 @@ def test_vision_token_roundtrip_and_host_selection():
     assert _as_frames(torch.zeros(2, 3 * 257), 256).shape == (2, 3, 257)  # vision_generation.py:219-221
     with pytest.raises(_lib.LwmError):
         _as_frames(torch.zeros(300), 256)
-
-
-@pytest.mark.skipif(not os.path.exists("/root/reference/lwm/llama.py"), reason="reference tree only in the build container")
-def test_reference_functions_still_reproduce_the_fixtures(tmp_path):
-    """re-run the generator (executes the reference's functions) into a scratch copy and compare with the committed files"""
-    code = ("import sys, os, numpy as np; sys.path.insert(0, %r); import make_golden_next_rows_from_reference as m; "
-            "m.ROOT = %r; os.makedirs(os.path.join(m.ROOT, 'tests', 'golden')); m.make_rope(); m.make_vision_tokens()"
-            % (os.path.join(ROOT, "tools"), str(tmp_path)))
-    r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=300)
-    assert r.returncode == 0, r.stderr[-2000:]
-    for name in ("rope_reference.npz", "vision_tokens_reference.npz"):
-        a, b = np.load(os.path.join(GOLD, name)), np.load(os.path.join(str(tmp_path), "tests", "golden", name))
-        assert sorted(a.files) == sorted(b.files)
-        for k in a.files:
-            assert np.array_equal(a[k], b[k]), (name, k)
 
 
 def test_call_site_mask_helpers():
